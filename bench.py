@@ -2,7 +2,7 @@
 """Benchmark of the DiffSBDD denoising hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-gpu]
-                    [--workload fullatom|ca|inpaint]
+                    [--workload fullatom|ca|inpaint] [--dump-outputs DIR]
 
 metric : ligand atoms/s through the full DDPM sampling loop of the per-GPU batch.
 workload (BASELINE.json configs, SURVEY.md §8(d)):
@@ -19,6 +19,10 @@ e2e    : same metric through the public API from pinned HOST buffers, host->devi
                        GPU box), all host threads it can use, bounded sample per step, extrapolated linearly.
 --impl reference-gpu : the same ATen op sequence as the reference on the B200 (device='cuda', eager, reference-order DDPM
                        loop): the fair "beat this" number of SURVEY.md §8(d); bounded sample, extrapolated linearly.
+--dump-outputs DIR   : b200 arm: after the timed steps, writes what the sampler returned in the last timed step as
+                       DIR/<name>.npy (float32, integer arrays as float64; at most 64 MB, else a fixed seeded sample of
+                       rows).  The inputs are seeded, so two builds run with the same arguments can be compared output
+                       for output.
 """
 from __future__ import annotations
 
@@ -41,6 +45,7 @@ import torch  # noqa: E402
 
 METRIC = 'ligand_atoms_per_sec_500step_ddpm'
 UNIT = 'ligand atoms/s'
+DUMP_BYTES = 64 * 10**6      # --dump-outputs writes at most this much
 
 WORKLOADS = {
     # name: (BASELINE.json config index, batch, n_lig, n_pocket, density, norm_values, yml, full-atom?)
@@ -72,7 +77,13 @@ def parse_args():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--profile-calls', type=int, default=10)
     ap.add_argument('--cpu-sample-seconds', type=float, default=20.0)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='b200 arm: write the outputs of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     _, b, nl, npk, _, _, _, _ = WORKLOADS[args.workload]
     args.batch = b if args.batch is None else args.batch
     args.n_lig = nl if args.n_lig is None else args.n_lig
@@ -216,6 +227,24 @@ def l2_flush(buf):
     buf.add_(1.0)    # read+write 256 MiB > 126 MB L2
 
 
+def dump_outputs(arrays, out_dir, limit=DUMP_BYTES):
+    """Writes every tensor of ``arrays`` to ``out_dir/<name>.npy``: float32 (float64 stays float64, integers become
+    float64, exactly).  If together they exceed ``limit`` bytes, each array keeps the same fraction of its rows, picked
+    with a fixed seed: the same rows for the same shapes, so that dumps of two runs stay comparable row for row."""
+    out = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        out[name] = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in 'iub' else np.float32)
+    total = sum(a.nbytes for a in out.values())
+    budget = limit - 1024 * len(out)           # room for the .npy headers
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        if total > budget and len(a):
+            keep = len(a) * budget // total
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 # ---- reference arms: the oracle port of the reference's PyTorch path, on the host cores or eager on the GPU -----------
 def _reference_ddpm(args, device):
     from diffsbdd_b200 import synthetic as syn
@@ -350,7 +379,7 @@ def run_reference_gpu(args):
     dyn.calls = 0
     sampler = ClockSampler(torch.device(device))
     sampler.start()
-    times = [_reference_run(args, ddpm, cfg, density, args.batch, sub, device) for _ in range(max(1, min(args.steps, 5)))]
+    times = [_reference_run(args, ddpm, cfg, density, args.batch, sub, device) for _ in range(args.steps)]
     clocks = sampler.stop()
     per_call = sum(times) / dyn.calls
     n_calls = denoiser_calls(args)
@@ -423,14 +452,17 @@ def run_b200(args):
         torch.cuda.synchronize(device)
 
     def step_device():
+        """One sampling run; returns what the caller receives, by name."""
         step_no[0] += 1
         if inpaint:
-            xh_lig, _, _, _ = ddpm.inpaint({k: v.clone() for k, v in lig_dev.items()}, dict(pocket_dev), fixed_dev,
-                                           resamplings=args.resamplings, timesteps=args.inpaint_timesteps, center='ligand')
-            return xh_lig
+            out = ddpm.inpaint({k: v.clone() for k, v in lig_dev.items()}, dict(pocket_dev), fixed_dev,
+                               resamplings=args.resamplings, timesteps=args.inpaint_timesteps, center='ligand')
+            return dict(zip(('xh_lig', 'xh_pocket', 'lig_mask', 'pocket_mask'), out))
         # library path: this rank's shard + the final all_gather of the ligands (the only collective of the path)
-        xh_all, _, _ = sample_given_pocket_sharded(ddpm, dict(job_dev), n_lig_job, base_seed=1000 * step_no[0], timesteps=T)
-        return xh_all
+        xh_all, sizes_all, local = sample_given_pocket_sharded(ddpm, dict(job_dev), n_lig_job, base_seed=1000 * step_no[0],
+                                                               timesteps=T)
+        return dict(zip(('xh_lig_all', 'lig_sizes_all', 'xh_lig', 'xh_pocket', 'lig_mask', 'pocket_mask'),
+                        (xh_all, sizes_all) + tuple(local)))
 
     def step_e2e():
         pocket = {k: v.to(device, non_blocking=True) for k, v in pocket_host.items()}
@@ -445,13 +477,14 @@ def run_b200(args):
         return xh_lig.cpu(), lig_mask.cpu()
 
     def timed(fn, k):
-        """k steps between two events; returns (max over ranks of the total ms, per-rank total ms list)."""
+        """k steps between two events; returns (max over ranks of the total ms, per-rank total ms list, what the last
+        step returned)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
             l2_flush(flush_buf)
-            fn()
+            last = fn()
         e1.record()
         torch.cuda.synchronize(device)
         ms = torch.tensor([e0.elapsed_time(e1)], device=device)
@@ -461,14 +494,16 @@ def run_b200(args):
             dist.all_gather(allms, ms)
             per_rank = [float(m.item()) for m in allms]
         barrier()
-        return max(per_rank), per_rank
+        return max(per_rank), per_rank, last
 
     for _ in range(args.warmup):
         step_device()
     sampler = ClockSampler(device)
     sampler.start()
-    ms_total, per_rank_ms = timed(step_device, args.steps)
+    ms_total, per_rank_ms, last = timed(step_device, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)      # before anything else reuses the sampler's buffers
     clocks_by_rank = None
     if world > 1:      # every rank sampled its own GPU: the per-rank clocks / power / throttle reasons name the limiter of a slow rank
         allc = [None] * world
@@ -483,7 +518,7 @@ def run_b200(args):
     e2e = None
     if not args.no_e2e:
         step_e2e()
-        ms_e2e, _ = timed(step_e2e, args.steps)
+        ms_e2e, _, _ = timed(step_e2e, args.steps)
         h2d = sum(v.numel() * v.element_size() for v in pocket_host.values())
         if inpaint:
             h2d += sum(v.numel() * v.element_size() for v in lig_host.values()) + fixed_host.numel() * 4

@@ -1,7 +1,8 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (/root/reference, via
-oracle/ref_shim.py) on seeded synthetic inputs and weights. Build-container only.
+"""Generates tests/golden/*.npz, tests/golden/second_draw/*.npz, tests/golden/fp64/*.npz and
+tests/golden/state_dict_layout.json by running the UNMODIFIED reference (imported through oracle/ref_shim.py, which
+finds its sources through DIFFSBDD_REFERENCE) on seeded synthetic inputs and weights.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [name ...]
 
 Each fixture stores the forward arguments, the reference outputs of ``EGNNDynamics.forward``
 (dynamics.py:87-167), the edge list the reference built (dynamics.py:169-187), the config, the weight
@@ -85,8 +86,23 @@ CASES = {
 }
 
 
-def make_inputs(case):
-    cfg, n_lig, n_poc, seed, wseed, density, t_value, norm_values = CASES[case]
+# a second input draw (input seed 100) of three of the cases, written to second_draw/<case>.npz in the same format
+SECOND_DRAW = ('ragged_b3_l4', 'moad_emb8_h192_l3', 'reflect_sub2_nocut_l2')
+SECOND_DRAW_SEED = 100
+
+# cases whose reference outputs are also computed in fp64 (the module and the stored inputs in double), written to
+# fp64/<case>.npz: unlike fp32 outputs, these do not depend on the CPU and thread count beyond ~1e-15
+FP64_CASES = ('config1_n64_l4', 'ca_b3_l6', 'joint_b2_h128_l5', 'mean_joint_h128_l2', 'reflect_sub2_nocut_l2',
+              'noatt_notanh_l2', 'sin_emb8_joint_h128_l2')
+
+# modules whose state-dict layout (keys in order, shapes, keys that name one shared tensor) goes to state_dict_layout.json
+LAYOUT_CONFIGS = [CONFIG1, DynamicsConfig(update_pocket_coords=True, reflection_equivariant=True, hidden_nf=128),
+                  DynamicsConfig(edge_embedding_dim=8, hidden_nf=192, n_layers=2, attention=False)]
+
+
+def make_inputs(case, seed=None):
+    cfg, n_lig, n_poc, case_seed, wseed, density, t_value, norm_values = CASES[case]
+    seed = case_seed if seed is None else seed
     tv = 0.37 if t_value == 'scalar' else t_value
     inp = list(syn.synthetic_denoiser_inputs(cfg, n_lig, n_poc, seed=seed, density=density,
                                              t_value=tv, norm_values=norm_values))
@@ -95,12 +111,28 @@ def make_inputs(case):
     return cfg, wseed, tuple(inp)
 
 
+def tied_groups(state_dict):
+    """Groups of state-dict keys that hold one tensor (a parameter shared between modules)."""
+    by_ptr = {}
+    for k, v in state_dict.items():
+        by_ptr.setdefault(v.data_ptr(), []).append(k)
+    return [g for g in by_ptr.values() if len(g) > 1]
+
+
+def state_dict_layout(cfg):
+    net = ref_shim.load_reference().EGNNDynamics(device='cpu', act_fn=torch.nn.SiLU(), **cfg.kwargs())
+    sd = net.state_dict()
+    return {'cfg': cfg.kwargs(), 'params': [[k, list(v.shape)] for k, v in sd.items()], 'tied': tied_groups(sd)}
+
+
 def main():
+    """Arguments, if any, name what to regenerate: a case, second_draw/<case>, fp64/<case> or state_dict_layout."""
     only = sys.argv[1:]
-    for case in CASES:
-        if only and case not in only:
+    todo = [(case, case, None) for case in CASES] + [('second_draw/' + c, c, SECOND_DRAW_SEED) for c in SECOND_DRAW]
+    for name, case, seed in todo:
+        if only and name not in only:
             continue
-        cfg, wseed, inp = make_inputs(case)
+        cfg, wseed, inp = make_inputs(case, seed)
         sd = syn.synthetic_state_dict(cfg, wseed)
         margin = syn.min_cutoff_margin(cfg, inp[0], inp[1], inp[3], inp[4])
         assert margin > 1e-4, (case, margin)
@@ -108,8 +140,9 @@ def main():
         with torch.no_grad():
             out_a, out_r = net(*inp)
             edges = net.get_edges(inp[3], inp[4], inp[0][:, :3], inp[1][:, :3])
+        os.makedirs(os.path.dirname(os.path.join(OUT, name)), exist_ok=True)
         np.savez_compressed(
-            os.path.join(OUT, case + '.npz'),
+            os.path.join(OUT, name + '.npz'),
             xh_atoms=inp[0].numpy(), xh_residues=inp[1].numpy(), t=inp[2].numpy(),
             mask_atoms=inp[3].numpy(), mask_residues=inp[4].numpy(),
             out_atoms=out_a.numpy(), out_residues=out_r.numpy(),
@@ -117,8 +150,25 @@ def main():
             cfg=json.dumps(cfg.kwargs()), weight_seed=wseed,
             weight_checksum=syn.state_dict_checksum(sd), cutoff_margin=margin,
         )
-        print(f'{case}: N_L={len(inp[3])} N_P={len(inp[4])} E={edges.shape[1]} margin={margin:.2e} '
+        print(f'{name}: N_L={len(inp[3])} N_P={len(inp[4])} E={edges.shape[1]} margin={margin:.2e} '
               f'|vel|max={out_a[:, :3].abs().max():.3f} |h|max={out_a[:, 3:].abs().max():.3f}')
+    for case in FP64_CASES:
+        if only and 'fp64/' + case not in only:
+            continue
+        z = np.load(os.path.join(OUT, case + '.npz'))
+        cfg = DynamicsConfig(**json.loads(str(z['cfg'])))
+        net = ref_shim.build_reference_dynamics(cfg, syn.synthetic_state_dict(cfg, int(z['weight_seed']))).double()
+        inp = [torch.from_numpy(z[k]) for k in ('xh_atoms', 'xh_residues', 't', 'mask_atoms', 'mask_residues')]
+        with torch.no_grad():
+            out_a, out_r = net(*[x.double() if x.is_floating_point() else x for x in inp])
+        os.makedirs(os.path.join(OUT, 'fp64'), exist_ok=True)
+        np.savez_compressed(os.path.join(OUT, 'fp64', case + '.npz'), out_atoms=out_a.numpy(), out_residues=out_r.numpy())
+        print(f'fp64/{case}: |out|max={max(out_a.abs().max(), out_r.abs().max()):.3f}')
+    if not only or 'state_dict_layout' in only:
+        with open(os.path.join(OUT, 'state_dict_layout.json'), 'w') as f:
+            json.dump([state_dict_layout(cfg) for cfg in LAYOUT_CONFIGS], f, indent=1)
+            f.write('\n')
+        print('state_dict_layout:', len(LAYOUT_CONFIGS), 'modules')
 
 
 if __name__ == '__main__':

@@ -1,4 +1,6 @@
 """CPU: drop-in boundary — state-dict / constructor / façade contracts (SURVEY.md §8(b))."""
+import json
+import os
 from argparse import Namespace
 
 import pytest
@@ -10,20 +12,42 @@ from diffsbdd_b200.conditional_model import ConditionalDDPM
 from diffsbdd_b200.dynamics import EGNNDynamics
 from diffsbdd_b200.en_diffusion import EnVariationalDiffusion, DistributionNodes
 from diffsbdd_b200.lightning_modules import LigandPocketDDPM
-from oracle import ref_shim
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='/root/reference not mounted')
+def tied_groups(state_dict):
+    """Groups of state-dict keys that hold one tensor (as tests/golden/make_golden.py records them)."""
+    by_ptr = {}
+    for k, v in state_dict.items():
+        by_ptr.setdefault(v.data_ptr(), []).append(k)
+    return [g for g in by_ptr.values() if len(g) > 1]
+
+
+def reference_layout(cfg):
+    """State-dict layout of the reference module for ``cfg`` (tests/golden/state_dict_layout.json, written by
+    tests/golden/make_golden.py): keys in order with shapes, and the groups of keys that hold one shared tensor."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'state_dict_layout.json')) as f:
+        for entry in json.load(f):
+            if entry['cfg'] == cfg.kwargs():
+                return entry
+    raise KeyError(f'no reference layout recorded for {cfg}')
+
+
 @pytest.mark.parametrize('cfg', [CONFIG1, DynamicsConfig(update_pocket_coords=True, reflection_equivariant=True, hidden_nf=128),
                                  DynamicsConfig(edge_embedding_dim=8, hidden_nf=192, n_layers=2, attention=False)])
 def test_state_dict_is_interchangeable_with_reference_module(cfg):
-    ref = ref_shim.load_reference().EGNNDynamics(device='cpu', act_fn=torch.nn.SiLU(), **cfg.kwargs())
+    ref = reference_layout(cfg)
     mine = EGNNDynamics.from_config(cfg)
-    r, m = ref.state_dict(), mine.state_dict()
-    assert list(r) == list(m)
-    assert all(r[k].shape == m[k].shape for k in r)
-    mine.load_state_dict(r, strict=True)                # reference checkpoint -> this module
-    ref.load_state_dict(mine.state_dict(), strict=True)  # and back
+    assert [[k, list(v.shape)] for k, v in mine.state_dict().items()] == ref['params']
+    # a reference checkpoint (shared parameters stored under each of their keys) -> this module
+    g = torch.Generator().manual_seed(0)
+    r = {k: torch.randn(shape, generator=g) for k, shape in ref['params']}
+    for group in ref['tied']:
+        for k in group[1:]:
+            r[k] = r[group[0]]
+    mine.load_state_dict(r, strict=True)
+    m = mine.state_dict()                               # and back
+    assert list(m) == list(r) and all(torch.equal(m[k], r[k]) for k in r)
+    assert tied_groups(m) == ref['tied']
     if not cfg.reflection_equivariant:                  # shared last layer stays shared (egnn_new.py:78)
         q = mine.egnn.e_block_0.gcl_equiv
         assert q.coord_mlp._modules['4'].weight is q.cross_product_mlp._modules['4'].weight
@@ -87,7 +111,7 @@ def test_lightning_facade_builds_and_roundtrips_checkpoint(tmp_path):
     torch.save({'state_dict': model.state_dict(), 'hyper_parameters': _hparams()}, ckpt)
     again = LigandPocketDDPM.load_from_checkpoint(str(ckpt), map_location='cpu')
     for k, v in model.state_dict().items():
-        assert torch.equal(v, again.state_dict()[k])
+        assert torch.equal(v.cpu(), again.state_dict()[k])      # the denoiser of `model` lives on cuda when there is one
     ca = LigandPocketDDPM(**_hparams(rep='CA'))
     assert ca.aa_nf == 20 and ca.pocket_type_encoder['A'] == 0
     joint = LigandPocketDDPM(**_hparams(mode='joint'))
