@@ -321,7 +321,7 @@ static Workspace carve(const dsb_config& c, int64_t NL, int64_t NP, int64_t B, i
   ws.xagg = (float4*)take(sizeof(float4) * (N + 1));
   ws.velmean = (float4*)take(sizeof(float4) * (B + 1));
   ws.h = (float*)take(sizeof(float) * (size_t)(N + 1) * H);
-  ws.hT = (float*)take(sizeof(float) * (size_t)(N + 257) * H);      // also the 3xFP16 operand image of h (whole 128-row tiles, one spare)
+  ws.hT = (float*)take(sizeof(float) * (size_t)(N + 1) * H);
   ws.agg = (float*)take(sizeof(float) * (size_t)(N + 1) * H);
   ws.P = (float*)take(sizeof(float) * (size_t)(N + 1) * 6 * H);
   ws.deg = (int32_t*)take(sizeof(int32_t) * (N + 1));
@@ -789,8 +789,8 @@ int dsb_dynamics_forward(dsb_dynamics* dyn, const float* xh_atoms, const float* 
 #define DSB_TRY(expr) do { if (int e_ = (expr)) return e_; } while (0)
   const int mm = (tc_width_supported(H) && !c.sin_embedding) ? dyn->math_mode : 0;      // sin_embedding: fp32 FFMA kernels only
   const bool f16 = (mm & 8) != 0;
-  auto gemm = [&](const GemmArgs& ga, const TcImage& img, int n_tile_off = 0) -> int {
-    return ((mm & 1) && img.t_hi) ? launch_tc_node_gemm(dyn, ga, img, n_tile_off, f16, status, s) : launch_node_gemm(ga, s);
+  auto gemm = [&](const GemmArgs& ga, const TcImage& img) -> int {
+    return ((mm & 1) && img.t_hi) ? launch_tc_node_gemm(dyn, ga, img, f16, status, s) : launch_node_gemm(ga, s);
   };
 
   mark(KC_SETUP);
@@ -810,7 +810,6 @@ int dsb_dynamics_forward(dsb_dynamics* dyn, const float* xh_atoms, const float* 
   const int nq = nm * 2 * H, ldP = nq + 2 * H, nrecv = nm * H;
   const PView pv_gcl = {ws.P + nq, ldP}, pv_coord = {ws.P, ldP};
   const bool conditional = dm.n_coord_rows < dm.N;
-  static const bool no_fused_mlp = getenv("DSB_NO_FUSED_MLP") != nullptr;      // A/B timing switch (two node GEMMs instead)
   for (int l = 0; l < c.n_layers; ++l) {
     bool fused_block = false;
     for (int sub = 0; sub < c.inv_sublayers; ++sub) {
@@ -826,20 +825,20 @@ int dsb_dynamics_forward(dsb_dynamics* dyn, const float* xh_atoms, const float* 
       // node_model: h + W4 SiLU(W3 [h | agg/norm] + b3) + b4   (egnn_new.py:48-58)
       mark(KC_NODE_GEMM);
       const EquivW& Qb = dyn->w.eq[l];
-      if ((mm & 1) && sub == c.inv_sublayers - 1 && G.iW3.h_hi && G.iW4.h_hi && Qb.iW1.h_hi && !no_fused_mlp && tc_node_block_available(H, f16)) {
+      if ((mm & 1) && sub == c.inv_sublayers - 1 && tc_node_block_available(H, f16)) {
         // node_model and the merged first-layer GEMM of this block in one CTA-pair kernel (h converted to operand format once)
         DSB_TRY(launch_tc_node_block(dyn, dm, ws, G, Qb, ws.P, ldP, conditional ? dm.n_coord_rows : 0, conditional ? nrecv : 0, s));
-        launches += 2 + ((g_kernel_variants & 4) ? 1 : 0);      // GCL edge kernel + block kernel (+ the split-off GEMM)
+        launches += 2;      // GCL edge kernel + block kernel
         fused_block = true;
-      } else if ((mm & 1) && G.iW3.t_hi && G.iW4.t_hi && !no_fused_mlp) {
+      } else if (mm & 1) {
         DSB_TRY(launch_tc_node_mlp(dyn, dm, ws, G, f16, status, s));        // both layers in one kernel, hidden stays on chip
         launches += 2;
       } else {
         GemmArgs g2 = {ws.h, H, H, ws.agg, H, H, c.normalization_factor, G.W3, H, G.b3, nullptr, 0, ws.hT, H, dm.N, H, 1, nullptr, 0, 0, 0,
                        c.aggregation_mean ? ws.deg : nullptr};
-        DSB_TRY(gemm(g2, G.iW3));
+        DSB_TRY(launch_node_gemm(g2, s));
         GemmArgs g3 = {ws.hT, H, H, nullptr, 0, 0, 1.f, G.W4, H, G.b4, ws.h, H, ws.h, H, dm.N, H, 0, ws.agg, H, 0, 0};
-        DSB_TRY(gemm(g3, G.iW4));
+        DSB_TRY(launch_node_gemm(g3, s));
         launches += 3;
       }
     }
@@ -878,7 +877,7 @@ int dsb_set_programmatic_launch(int enable) {
 
 int dsb_set_kernel_variants(int variants) {
   const int old = dsb::g_kernel_variants;
-  if (variants >= 0) dsb::g_kernel_variants = variants & 7;
+  if (variants >= 0) dsb::g_kernel_variants = variants & 3;
   return old;
 }
 

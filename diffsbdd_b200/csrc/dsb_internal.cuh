@@ -84,7 +84,7 @@ struct Workspace {
   float4 *cent;                 // [B]
   float4 *xagg;                 // [N] raw segment sums of trans
   float4 *velmean;              // [B]
-  float *h, *hT, *agg, *P;      // [N][H], [N][H], [N][H], [N][6H] (Q block of the current layer | P block of the next GCL)
+  float *h, *hT, *agg, *P;      // [N][H], [N][H] (hidden layer of the fp32 node MLP), [N][H], [N][6H] (Q block of the current layer | P block of the next GCL)
   int32_t *deg, *row_ptr;       // [N], [N+1]
   int32_t *vrow_ptr, *vmap;     // [N+1], [Ecap + 3N]: receiver segments padded to multiples of kRowChunk rows (tensor-core edge kernels)
   int32_t *erow, *ecol;         // [Ecap]
@@ -220,8 +220,7 @@ void launch_pack_b_image_f16(float* hi, float* lo, const float* src, int lds, in
 void launch_absmax(const float* src, int lds, int scol, int n_rows, int K, unsigned* out);
 int configure_tc_kernels(int H);
 bool tc_width_supported(int H);     // hidden_nf values with tensor-core kernels (128, 192, 256)
-int launch_tc_node_gemm(const dsb_dynamics* d, const GemmArgs& g, const TcImage& w, int n_tile_off, bool f16, int32_t* status,
-                        cudaStream_t s);
+int launch_tc_node_gemm(const dsb_dynamics* d, const GemmArgs& g, const TcImage& w, bool f16, int32_t* status, cudaStream_t s);   // C = A1 W + bias only
 int launch_tc_node_mlp(const dsb_dynamics* d, const Dims& dm, const Workspace& ws, const GclW& w, bool f16, int32_t* status, cudaStream_t s);
 bool tc_node_block_available(int H, bool f16);
 int launch_tc_node_block(const dsb_dynamics* d, const Dims& dm, const Workspace& ws, const GclW& w, const EquivW& q, float* P, int ldp,
@@ -258,25 +257,9 @@ __device__ __forceinline__ f32x2 silu2(f32x2 u) {
   return mul2(u, pk2(rcp_approx(a), rcp_approx(b)));
 }
 
-// SiLU of four values with TWO reciprocals instead of four: the 16-lane XU pipe (MUFU: 8 issue cycles per warp instruction
+// SiLU of four values with ONE reciprocal instead of four: the 16-lane XU pipe (MUFU: 8 issue cycles per warp instruction
 // and sub-partition) is the busiest pipe of the edge kernels (2 SiLU per edge element = 4 MUFU), the FMA pipe is not.
-//   d_i = 1 + 2^{t_i},  r = 1 / (d_a d_b)  ->  1/d_a = r d_b,  1/d_b = r d_a          (elements 0,2 and 1,3 are paired)
-// The exponent argument is clamped to 64 (pre-activation >= -44.4, where SiLU(x) = x e^x is below 3e-18 in magnitude) so that
-// neither d nor, harmfully, the product can reach inf next to a finite partner (0 * inf); a product of exactly 2^128 gives
-// r = 0 and both results 0.  Relative error ~4e-7 (one rcp.approx and two roundings more than silu_f).
-__device__ __forceinline__ void silu4(f32x2& u01, f32x2& u23) {
-  const f32x2 c = pk2(-1.4426950408889634f, -1.4426950408889634f), one = pk2(1.0f, 1.0f);
-  float t0, t1, t2, t3;
-  upk2(mul2(u01, c), t0, t1); upk2(mul2(u23, c), t2, t3);
-  const f32x2 d01 = add2(pk2(ex2_approx(fminf(t0, 64.f)), ex2_approx(fminf(t1, 64.f))), one);
-  const f32x2 d23 = add2(pk2(ex2_approx(fminf(t2, 64.f)), ex2_approx(fminf(t3, 64.f))), one);
-  float p0, p1;
-  upk2(mul2(d01, d23), p0, p1);
-  const f32x2 r = pk2(rcp_approx(p0), rcp_approx(p1));
-  u01 = mul2(u01, mul2(r, d23));
-  u23 = mul2(u23, mul2(r, d01));
-}
-// The same with ONE reciprocal for the four values: r = 1 / (d_0 d_1 d_2 d_3), 1/d_0 = r (d_1 d_3) d_2 ... arranged on pairs:
+// With d_i = 1 + 2^{t_i}: r = 1 / (d_0 d_1 d_2 d_3), 1/d_0 = r (d_1 d_3) d_2 ... arranged on pairs:
 //   p = d01 * d23 = (d_0 d_2, d_1 d_3);  r = 1 / (p.x p.y);  (r p.y, r p.x) = (1/(d_0 d_2), 1/(d_1 d_3));  times d23 -> 1/d01,
 //   times d01 -> 1/d23.  5 MUFU per 4 values.  Exponent argument clamped to 31 (four factors below 2^31 + 1 cannot overflow;
 // pre-activation >= -21.5, where |SiLU(x)| < 1e-8 and the clamp changes it by < 5e-9).  Relative error ~6e-7.
@@ -293,18 +276,6 @@ __device__ __forceinline__ void silu4q(f32x2& u01, f32x2& u23) {
   const f32x2 rr = mul2(pk2(r, r), pk2(p1, p0));  // (1 / (d0 d2), 1 / (d1 d3)); broadcast and swapped pair are operand modifiers
   u01 = mul2(w01, rr);
   u23 = mul2(w23, rr);
-}
-#ifndef DSB_SILU_PAIR
-#define DSB_SILU_PAIR 3          // bit 0: producers, bit 1: epilogues of the tensor-core edge kernels use silu4
-#endif
-#ifndef DSB_SILU_QUAD
-#define DSB_SILU_QUAD 3          // bit 0: producers, bit 1: epilogues use silu4q (one reciprocal per four values) instead
-#endif
-template <bool PAIR, bool QUAD = false>
-__device__ __forceinline__ void silu_pair(f32x2& u01, f32x2& u23) {
-  if constexpr (QUAD) silu4q(u01, u23);
-  else if constexpr (PAIR) silu4(u01, u23);
-  else { u01 = silu2(u01); u23 = silu2(u23); }
 }
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {

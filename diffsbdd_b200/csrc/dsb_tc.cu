@@ -5,8 +5,7 @@
 //   tc_edge_kernel<1,..>   — EquivariantUpdate.coord_model                  (egnn_new.py:96-116)
 //                            PAIR = true (3xFP16 default): CTA pairs, tcgen05 cta_group::2, second-layer weights resident
 //   tc_node_block_kernel   — GCL.node_model + the merged first-layer GEMM that consumes the new h, CTA pairs (egnn_new.py:48-58)
-//   tc_pair_gemm_kernel    — that GEMM as a separate CTA-pair kernel fed by an operand image of h (optional split)
-//   tc_node_gemm_kernel    — C = act([A1 | A2/div] @ W + bias) (+R)         (first block's first layer; single-CTA fallback)
+//   tc_node_gemm_kernel    — C = A @ W + bias                               (first block's first layer; single-CTA merged GEMM)
 //   tc_node_mlp_kernel     — node_model alone, single CTA                   (3xTF32 / dsb_set_kernel_variants(0))
 //
 // One persistent CTA per SM, warp-specialised (see dsb_tc.cuh); the roles of the edge kernels:
@@ -24,12 +23,6 @@
 namespace dsb {
 using namespace tc;
 
-
-// tuning switch (profiles/build_variants.py): 1 = producers of the node kernels issue their prefetch loads before the proxy fence
-#ifndef DSB_LOADS_BEFORE_FENCE
-#define DSB_LOADS_BEFORE_FENCE 0
-#endif
-constexpr bool kLoadsBeforeFence = DSB_LOADS_BEFORE_FENCE != 0;
 
 // =====================================================================================================
 // weight images: B[n][k] (= the reference's own [out][in] Linear layout) split into hi/lo and laid out as
@@ -157,12 +150,10 @@ __device__ __forceinline__ void tma_role(Control* ctl, char* stages, const float
 // node GEMM
 // =====================================================================================================
 struct TcGemmArgs {
-  const float* A1; int lda1; int K1;
-  const float* A2; int lda2; int K2; float div2; const int32_t* deg2;     // deg2 != nullptr: per-row divisor max(deg2[m], 1) ('mean')
+  const float* A; int lda; int K;
   const float* Bhi; const float* Blo;        // [Nn/256][K/32][8192]
-  const float* bias; const float* R; int ldr;
-  float* C; int ldc; int M; int Nn; int act;
-  float* Z; int ldz;
+  const float* bias;
+  float* C; int ldc; int M; int Nn;
   int dead_mt; int dead_nt;                    // tiles with m-tile >= dead_mt and n-tile < dead_nt are skipped (dead_nt == 0: none)
   float inv_scale;                             // 3xFP16: 1 / (X_SCALE * weight scale); 1 for 3xTF32
   int32_t* status;
@@ -195,7 +186,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
   const int n_tiles = tm.n_live;
   const int n_my = ((int)blockIdx.x < n_tiles) ? (n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
   if (n_my == 0) return;
-  const int K = g.K1 + g.K2, halves = K / TKC, chunks = F16 ? halves / 2 : halves;
+  const int halves = g.K / TKC, chunks = F16 ? halves / 2 : halves;
   const bool gprof = (tc_debug() & 512) && blockIdx.x == 0;
   const long long k0 = gprof ? tc_clock() : 0;
   pdl_trigger();
@@ -206,7 +197,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
 
   if (warp < EPI_WARPS) {
     // Epilogue.  tcgen05.ld gives each thread one accumulator ROW; storing rows directly would make every
-    // STG.128 / residual LDG.128 touch 32 different rows (32 L1 wavefronts per 512 bytes).  Each 32x32 block is
+    // STG.128 touch 32 different rows (32 L1 wavefronts per 512 bytes).  Each 32x32 block is
     // therefore transposed through a per-warp shared buffer so that 8 lanes cover 128 contiguous bytes of one row
     // (4 rows = 4 wavefronts per instruction).
     float* T = reinterpret_cast<float*>(cv.extra) + warp * (32 * GEMM_T_STRIDE);
@@ -222,19 +213,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
       const long long e1 = gprof ? tc_clock() : 0;
       if (gprof && threadIdx.x == 0) atomicAdd(&g_tc_prof[17], (unsigned long long)(e1 - (it == 0 ? k1 : e0)));   // epilogue waits for the accumulator
       const uint32_t taddr = ctl->tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(a * ACC_STRIDE);
-      // residual rows of column block cb+1 are requested while block cb is processed (two register sets, loop unrolled by 2)
-      auto load_res = [&](int cb, float4 (&rr)[8]) {
+#pragma unroll 1
+      for (int cb = 0; cb < ((tc_debug() & 4) ? 0 : TN / 32); ++cb) {
         const int n = n0 + cb * 32 + tc4;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int row = m0 + warp * 32 + 4 * i + tr;
-          rr[i] = row < g.M ? *reinterpret_cast<const float4*>(g.R + (size_t)row * g.ldr + n) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      };
-      auto do_block = [&](int cb, const float4 (&rr)[8]) {
-        const int n = n0 + cb * 32 + tc4;
-        float4 bias = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (g.bias) bias = __ldg(reinterpret_cast<const float4*>(g.bias + n));
+        const float4 bias = __ldg(reinterpret_cast<const float4*>(g.bias + n));
         float v[32];
         tmem_ld32(taddr + cb * 32, v);
 #pragma unroll
@@ -251,26 +233,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
             f32x2 x01 = pk2(x.x, x.y), x23 = pk2(x.z, x.w);
             if (F16) { x01 = fma2(x01, ip, b01); x23 = fma2(x23, ip, b23); }
             else { x01 = add2(x01, b01); x23 = add2(x23, b23); }
-            if (g.act == 1) { x01 = silu2(x01); x23 = silu2(x23); }
-            if (g.R) { x01 = add2(pk2(rr[i].x, rr[i].y), x01); x23 = add2(pk2(rr[i].z, rr[i].w), x23); }
             float4 o;
             upk2(x01, o.x, o.y); upk2(x23, o.z, o.w);
-            if (!(tc_debug() & 32)) {
-              *reinterpret_cast<float4*>(g.C + (size_t)row * g.ldc + n) = o;
-              if (g.Z) *reinterpret_cast<float4*>(g.Z + (size_t)row * g.ldz + n) = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
+            if (!(tc_debug() & 32)) *reinterpret_cast<float4*>(g.C + (size_t)row * g.ldc + n) = o;
           }
         }
         __syncwarp();
-      };
-      float4 ra[8], rb[8];
-      if (g.R) load_res(0, ra);
-#pragma unroll 1
-      for (int cb = 0; cb < ((tc_debug() & 4) ? 0 : TN / 32); cb += 2) {
-        if (g.R) load_res(cb + 1, rb);
-        do_block(cb, ra);
-        if (g.R && cb + 2 < TN / 32) load_res(cb + 2, ra);
-        do_block(cb + 1, rb);
       }
       if (gprof && threadIdx.x == 0) atomicAdd(&g_tc_prof[18], (unsigned long long)(tc_clock() - e1));             // epilogue work of one tile
       tc_fence_before();
@@ -288,13 +256,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
       for (int i = 0; i < 4; ++i) {
         const int m = m0 + 16 * pw + 4 * sr + i;
         float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (m < g.M && !(tc_debug() & 2)) {
-          if (k < g.K1) {
-            x = *reinterpret_cast<const float4*>(g.A1 + (size_t)m * g.lda1 + k);
-          } else {
-            x = *reinterpret_cast<const float4*>(g.A2 + (size_t)m * g.lda2 + (k - g.K1));     // divided by div2 when staged
-          }
-        }
+        if (m < g.M && !(tc_debug() & 2)) x = *reinterpret_cast<const float4*>(g.A + (size_t)m * g.lda + k);
         v[i] = x;
       }
     };
@@ -316,29 +278,17 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
       const int s = gc & 1;
       mbar_wait(&ctl->empty[s], ((gc >> 1) & 1) ^ 1);
       char* st = cv.stages + (size_t)s * G::STAGE_BYTES;
-      const int kc = q % chunks;
 #pragma unroll
-      for (int h = 0; h < HPC; ++h) {
-        const bool second = (g.div2 != 1.0f || g.deg2) && (kc * HPC + h) * TKC + 4 * pc >= g.K1;      // columns of A2: exact division here,
-#pragma unroll                                                                              // not at load time (keeps the loads in flight)
-        for (int i = 0; i < 4; ++i) {
-          float4 x = buf[h][i];
-          if (second) {
-            const int m = tile_m0(q / chunks) + 16 * pw + 4 * sr + i;
-            const float dv = g.deg2 ? (float)max(m < g.M ? g.deg2[m] : 1, 1) : g.div2;
-            x.x = __fdiv_rn(x.x, dv); x.y = __fdiv_rn(x.y, dv); x.z = __fdiv_rn(x.z, dv); x.w = __fdiv_rn(x.w, dv);
-          }
-          store_piece<F16>(st, 16 * pw + 4 * sr + i, h, pc, x);
-        }
-      }
+      for (int h = 0; h < HPC; ++h)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) store_piece<F16>(st, 16 * pw + 4 * sr + i, h, pc, buf[h][i]);
       // fence.proxy.async waits for every outstanding load of the thread (FENCE.VIEW.ASYNC stalls on the long scoreboard,
       // profiles/r1 source view): loads issued BEFORE it put a full L2 round trip between the stores and the arrive, on the
       // MMA thread's critical path (wait-X 1.8 k cycles/chunk).  Issue the next loads after the hand-off instead.
-      if (kLoadsBeforeFence && q + 2 < total) load_chunk(q + 2, buf);
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(&ctl->full_x[s]);
-      if (!kLoadsBeforeFence && q + 2 < total) load_chunk(q + 2, buf);
+      if (q + 2 < total) load_chunk(q + 2, buf);
       ++gc;
     };
     float4 bufA[HPC][4], bufB[HPC][4];
@@ -374,12 +324,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_gemm_kernel(TcGemmArgs 
 
 // =====================================================================================================
 // fused node MLP (egnn_new.py:48-58): h <- h + W4 SiLU(W3 [h | agg/norm] + b3) + b4 for one 128-row tile per CTA.
-// Phase 1 is the node GEMM above (producers build the A operand from h and agg, K = 2H, accumulator 0).  Its epilogue does
-// not go to global memory: the four epilogue warps apply bias + SiLU to the accumulator and write the result, already split
-// and swizzled, into the A slots of the stage ring, i.e. they ARE the producers of phase 2 (K = H, accumulator 1), whose
-// weight chunks the bulk-copy thread streams right behind those of phase 1.  The phase-2 epilogue adds bias and residual,
-// stores the new h in place (rows are private to the CTA) and re-arms the aggregate.  One launch and one [N,H] round trip
-// through global memory less than two node GEMMs.
+// Phase 1 is a node GEMM as above, its producers build the A operand from h and agg/norm (K = 2H, accumulator 0).  Its
+// epilogue does not go to global memory: the four epilogue warps apply bias + SiLU to the accumulator and write the result,
+// already split and swizzled, into the A slots of the stage ring, i.e. they ARE the producers of phase 2 (K = H,
+// accumulator 1), whose weight chunks the bulk-copy thread streams right behind those of phase 1.  The phase-2 epilogue adds
+// bias and residual, stores the new h in place (rows are private to the CTA) and re-arms the aggregate.  One launch and one
+// [N,H] round trip through global memory less than two node GEMMs.
 // =====================================================================================================
 struct TcMlpArgs {
   const float* h; int ldh;                      // A1 of phase 1, residual of phase 2, output (in place)
@@ -546,11 +496,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_mlp_kernel(TcMlpArgs g)
           store_piece<F16>(st, 16 * pw + 4 * sr + i, h, pc, x);
         }
       }
-      if (kLoadsBeforeFence && j + 2 < total) load_chunk(j + 2, buf);
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(&ctl->full_x[s]);
-      if (!kLoadsBeforeFence && j + 2 < total) load_chunk(j + 2, buf);      // see tc_node_gemm_kernel
+      if (j + 2 < total) load_chunk(j + 2, buf);      // after the fence: see tc_node_gemm_kernel
     };
     float4 bufA[HPC][4], bufB[HPC][4];
     load_chunk(0, bufA);
@@ -610,7 +559,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_mlp_kernel(TcMlpArgs g)
 // weight columns (B split along N): 32 KB per k-chunk and CTA.
 // Barriers: full_a / epi_done / w_peer live in the leader (cluster rank 0), whose MMA thread issues for both CTAs; the peer's
 // warps arrive through the cluster address space; e0 / e3 / empty_w / acc_full are multicast commits.  A slot is written four
-// times per item (phase-1 chunks 0..3, chunks 4..7, hid, new h; three without phase 3): full_a completes once per write.
+// times per item (phase-1 chunks 0..3, chunks 4..7, hid, new h): full_a completes once per write.
 // A parity wait can only tell "the phase I expect" from "the next one", so every waiter follows its barrier phase by phase:
 // the producers' second write waits for e0 (phase-1 chunk 0..3 read), their first write of the NEXT item for e3 (last
 // phase-3 read), one completion per item each; the epilogue's writes are ordered by acc_full (all MMAs of the phase done).
@@ -629,8 +578,6 @@ struct TcBlockArgs {
   float inv3, inv4, invq, s4;                 // 1 / weight scale per image (powers of two); s4 = 1 / inv4
   float* P; int ldp; int Nn;
   int M; int dead_mt; int dead_nt;            // column tiles < dead_nt are not needed for row tiles >= dead_mt
-  char* himg;                                 // != nullptr: no phase 3; the new h is also written as a 3xFP16 operand image,
-                                              // [row tile][k-chunk][hi | lo: 128 rows x 128 B, SWIZZLE_128B], for tc_pair_gemm_kernel
 };
 struct BlockControl {
   uint64_t full_a[4], e0[4], e3[4];
@@ -745,7 +692,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
             const float4 bb = __ldg(reinterpret_cast<const float4*>(g.b3 + cb * 32 + 4 * p8));
             f32x2 x01 = fma2(pk2(v[4 * p8], v[4 * p8 + 1]), ip, pk2(bb.x, bb.y));
             f32x2 x23 = fma2(pk2(v[4 * p8 + 2], v[4 * p8 + 3]), ip, pk2(bb.z, bb.w));
-            silu_pair<true, true>(x01, x23);
+            silu4q(x01, x23);
             float4 x;
             upk2(x01, x.x, x.y); upk2(x23, x.z, x.w);
             store_piece<true>(st, myrow, cb & 1, p8, x);
@@ -760,45 +707,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(l_epi_done + 8u * (u & 1));
         ++u;
-      }
-      if (g.himg) {
-        // ---- phase-2 epilogue without phase 3: new h = acc * inv4 to global memory (in place), as fp32 and as the operand
-        // image the merged GEMM will bulk-copy; aggregate re-armed.  8 lanes cover 128 contiguous bytes of a row (fp32) resp.
-        // 64 bytes of its swizzled image row.
-        mbar_wait(&ctl->acc_full[u & 1], (u >> 1) & 1);
-        tc_fence_after();
-        const uint32_t taddr = tbase + (uint32_t)((u & 1) * ACC_STRIDE);
-        const f32x2 ip = pk2(g.inv4, g.inv4);
-        char* const img = g.himg + (size_t)(2 * item_mp(it) + rank) * (size_t)(NSLOT * SLOT_BYTES);
-#pragma unroll 1
-        for (int cb = 0; cb < H / 32; ++cb) {
-          const int n = cb * 32 + tc4;
-          float v[32];
-          tmem_ld32(taddr + cb * 32, v);
-#pragma unroll
-          for (int q = 0; q < 8; ++q)
-            *reinterpret_cast<float4*>(T + lane * GEMM_T_STRIDE + 4 * q) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-          __syncwarp();
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int rl = 4 * i + tr;
-            const int row = m0 + warp * 32 + rl;
-            const float4 x = *reinterpret_cast<const float4*>(T + rl * GEMM_T_STRIDE + tc4);
-            float4 o;
-            upk2(mul2(pk2(x.x, x.y), ip), o.x, o.y); upk2(mul2(pk2(x.z, x.w), ip), o.z, o.w);
-            if (row < g.M) {
-              *reinterpret_cast<float4*>(g.h + (size_t)row * g.ldh + n) = o;
-              *reinterpret_cast<float4*>(g.agg + (size_t)row * g.ldagg + n) = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-            store_piece<true>(img + (size_t)(cb >> 1) * SLOT_BYTES, warp * 32 + rl, cb & 1, lane & 7, o);    // rows beyond M: finite, never used
-          }
-          __syncwarp();
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(l_epi_done + 8u * (u & 1));
-        ++u;
-        continue;
       }
       // ---- phase-2 epilogue: new h = acc * inv4 (the accumulator started from (h + b4) * s4).  First the phase-3 A operand
       // (fourth write of a slot; phase 3 starts as soon as all four slots are handed over), then the global side: h in place,
@@ -989,9 +897,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
         return tmem + (uint32_t)((u & 1) * ACC_STRIDE);
       };
       auto end_use = [&]() { umma_commit_2cta(&ctl->acc_full[u & 1]); ++u; };
-      const uint32_t wpi = g.himg ? 3u : 4u;       // writes of a slot (= completions of its full_a) per item
       for (int it = 0; it < n_items; ++it) {
-        const uint32_t fa = (uint32_t)it * wpi;     // full_a completions before this item: write k of the item has parity (fa + k) & 1
+        const uint32_t fa = (uint32_t)it * 4u;      // full_a completions before this item (4 slot writes per item): write k has parity (fa + k) & 1
         ph = 0;
         uint32_t d = begin_use();
         for (int kc = 0; kc < C1; ++kc) chunk(d, kc % NSLOT, (fa + (kc < NSLOT ? 0u : 1u)) & 1u, true, kc == 0, kc < NSLOT ? &ctl->e0[kc] : nullptr);     // slot writes 1, 2
@@ -1000,9 +907,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
         d = begin_use();
         mbar_wait_cluster(&ctl->pre_done, (uint32_t)it & 1u);          // the accumulator holds the residual in both CTAs
         tc_fence_after();
-        for (int kc = 0; kc < C2; ++kc) chunk(d, kc, (fa + 2u) & 1u, true, false, g.himg ? &ctl->e3[kc] : nullptr);       // slot write 3 (hid); accumulates onto the residual (no phase 3: last read of the slot)
+        for (int kc = 0; kc < C2; ++kc) chunk(d, kc, (fa + 2u) & 1u, true, false, nullptr);       // slot write 3 (hid); accumulates onto the residual
         end_use();
-        const int nt0 = g.himg ? ntn : item_nt0(it);
+        const int nt0 = item_nt0(it);
         ph = 2;
         for (int nt = nt0; nt < ntn; ++nt) {
           d = begin_use();
@@ -1021,7 +928,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
     } else if (lane == 0) {
       // peer CTA: forward "my weight half of chunk gw has landed" to the leader
       uint32_t total = 0;
-      for (int it = 0; it < n_items; ++it) total += C1 + C2 + (g.himg ? 0u : (uint32_t)(ntn - item_nt0(it)) * C2);
+      for (int it = 0; it < n_items; ++it) total += C1 + C2 + (uint32_t)(ntn - item_nt0(it)) * C2;
       for (uint32_t gw = 0; gw < total; ++gw) {
         mbar_wait(&ctl->full_w[gw & 1], (gw >> 1) & 1);
         mbar_arrive_cluster(l_w_peer + 8u * (gw & 1));
@@ -1044,7 +951,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
       for (int it = 0; it < n_items; ++it) {
         for (int kc = 0; kc < C1; ++kc) load(g.W3hi, g.W3lo, kc);
         for (int kc = 0; kc < C2; ++kc) load(g.W4hi, g.W4lo, kc);
-        for (int nt = g.himg ? ntn : item_nt0(it); nt < ntn; ++nt)
+        for (int nt = item_nt0(it); nt < ntn; ++nt)
           for (int kc = 0; kc < C2; ++kc) load(g.Wqhi + (size_t)nt * C2 * G::B_CHUNK_FLOATS, g.Wqlo + (size_t)nt * C2 * G::B_CHUNK_FLOATS, kc);
       }
     }
@@ -1054,183 +961,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_node_block_kernel(TcBlockArg
 }
 
 // =====================================================================================================
-// CTA-pair GEMM from an operand image: C[M][Nn] = h Wq + bq, A = the 3xFP16 image of h written by tc_node_block_kernel.
-// No producer warps: a k-chunk of A (hi | lo, 32 KB: this CTA's 128 rows) and this CTA's half of the weight columns (32 KB)
-// arrive by bulk copy into a 3-deep ring; the leader issues M = 256 MMAs for the pair.  Work items = live (row-tile pair,
-// column tile) combinations dealt round-robin to the 74 pairs: unlike the phase 3 of the fused kernel (one item of 16-24
-// k-chunks per pair, 24 pairs idle, the ligand rows' items 50 % longer than the rest) every pair gets ~3 items of 4 k-chunks.
-// =====================================================================================================
-struct TcPairGemmArgs {
-  const char* himg;                           // [row tile][H/64][hi | lo]
-  const float *Whi, *Wlo; const float* bias; float inv;
-  float* C; int ldc; int M; int Nn; int dead_mt; int dead_nt;
-};
-struct PairGemmControl {
-  uint64_t full[3], peer[3], empty[3];
-  uint64_t acc_full[2], epi_done[2];
-  uint32_t tmem_base, pad;
-};
-constexpr int PG_STAGES = 3;
-template <int H> constexpr size_t pair_gemm_smem_bytes() {
-  return 1024 + (size_t)PG_STAGES * (2 * A_CHUNK_BYTES + (size_t)H * 128) + kControlBytes + sizeof(float) * EPI_WARPS * 32 * GEMM_T_STRIDE;
-}
-constexpr int PG_THREADS = (EPI_WARPS + 2) * 32;      // 4 epilogue warps, MMA warp, bulk-copy warp
-
-template <int H>
-__global__ void __launch_bounds__(PG_THREADS, 1) tc_pair_gemm_kernel(TcPairGemmArgs g) {
-  using G = Geo<H>;
-  constexpr int C2 = H / TKC16;
-  constexpr int SLOT_BYTES = 2 * A_CHUNK_BYTES, HB = (H / 2) * 128, STAGE = SLOT_BYTES + 2 * HB;
-  constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(H >> 3) << 17) | ((uint32_t)((2 * TM) >> 4) << 24);
-  constexpr int PG_MMA = EPI_WARPS;                // warp PG_MMA + 1 issues the bulk copies
-  extern __shared__ uint8_t smem_raw[];
-  char* const ring = reinterpret_cast<char*>(smem_raw) + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  PairGemmControl* ctl = reinterpret_cast<PairGemmControl*>(ring + PG_STAGES * STAGE);
-  float* const Tall = reinterpret_cast<float*>(reinterpret_cast<char*>(ctl) + kControlBytes);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int rank = (int)cluster_ctarank(), pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-  const int ntm = (g.M + TM - 1) / TM, nmp = (ntm + 1) / 2, ntn = g.Nn / H;
-  // live items: row-tile pairs [0, dmp) x all column tiles, then [dmp, nmp) x column tiles [dead_nt, ntn)
-  const int dmp = g.dead_nt > 0 ? min((g.dead_mt + 1) / 2, nmp) : nmp;
-  const int nA = dmp * ntn, n_live = nA + (nmp - dmp) * (ntn - g.dead_nt);
-  auto item = [&](int t, int& mp, int& nt) {
-    if (t < nA) { mp = t / ntn; nt = t - mp * ntn; }
-    else { const int w = ntn - g.dead_nt, v = t - nA; mp = dmp + v / w; nt = g.dead_nt + (v - (v / w) * w); }
-  };
-  pdl_trigger();
-  if (threadIdx.x == 0) {
-    for (int k = 0; k < PG_STAGES; ++k) { mbar_init(&ctl->full[k], 1); mbar_init(&ctl->peer[k], 1); mbar_init(&ctl->empty[k], 1); }
-    for (int k = 0; k < 2; ++k) { mbar_init(&ctl->acc_full[k], 1); mbar_init(&ctl->epi_done[k], 2 * EPI_WARPS); }
-    fence_barrier_init();
-  }
-  __syncthreads();
-  if (warp == PG_MMA) tmem_alloc2(&ctl->tmem_base, 512);
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  pdl_wait();
-  const int n_my = pair < n_live ? (n_live - pair + npairs - 1) / npairs : 0;
-  const uint32_t l_epi_done = leader_addr(&ctl->epi_done[0]), l_peer = leader_addr(&ctl->peer[0]);
-
-  if (warp < EPI_WARPS) {
-    float* T = Tall + warp * (32 * GEMM_T_STRIDE);
-    const int tr = lane >> 3, tc4 = (lane & 7) * 4;
-    const uint32_t tbase = ctl->tmem_base + ((uint32_t)(warp * 32) << 16);
-    const f32x2 ip = pk2(g.inv, g.inv);
-    for (int j = 0; j < n_my; ++j) {
-      int mp, nt;
-      item(pair + j * npairs, mp, nt);
-      const int m0 = (2 * mp + rank) * TM;
-      mbar_wait(&ctl->acc_full[j & 1], (j >> 1) & 1);
-      tc_fence_after();
-      const uint32_t taddr = tbase + (uint32_t)((j & 1) * ACC_STRIDE);
-#pragma unroll 1
-      for (int cb = 0; cb < H / 32; ++cb) {
-        const int n = nt * H + cb * 32 + tc4;
-        const float4 bias = __ldg(reinterpret_cast<const float4*>(g.bias + n));
-        float v[32];
-        tmem_ld32(taddr + cb * 32, v);
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          *reinterpret_cast<float4*>(T + lane * GEMM_T_STRIDE + 4 * q) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-        __syncwarp();
-        const f32x2 b01 = pk2(bias.x, bias.y), b23 = pk2(bias.z, bias.w);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int rl = 4 * i + tr;
-          const int row = m0 + warp * 32 + rl;
-          const float4 x = *reinterpret_cast<const float4*>(T + rl * GEMM_T_STRIDE + tc4);
-          float4 o;
-          upk2(fma2(pk2(x.x, x.y), ip, b01), o.x, o.y); upk2(fma2(pk2(x.z, x.w), ip, b23), o.z, o.w);
-          if (row < g.M) *reinterpret_cast<float4*>(g.C + (size_t)row * g.ldc + n) = o;
-        }
-        __syncwarp();
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(l_epi_done + 8u * (uint32_t)(j & 1));
-    }
-  } else if (warp == PG_MMA) {
-    if (lane == 0 && rank == 0) {
-      const uint32_t tmem = ctl->tmem_base;
-      uint32_t gw = 0;
-      for (int j = 0; j < n_my; ++j) {
-        mbar_wait_cluster(&ctl->epi_done[j & 1], ((j >> 1) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t d = tmem + (uint32_t)((j & 1) * ACC_STRIDE);
-        for (int kc = 0; kc < C2; ++kc, ++gw) {
-          const int s = gw % PG_STAGES;
-          const uint32_t par = (gw / PG_STAGES) & 1;
-          mbar_wait(&ctl->full[s], par);
-          mbar_wait_cluster(&ctl->peer[s], par);
-          tc_fence_after();
-          const uint32_t xhi = smem_u32(ring + (size_t)s * STAGE), xlo = xhi + A_CHUNK_BYTES;
-          const uint32_t whi = xhi + SLOT_BYTES, wlo = whi + HB;
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks) {
-            const uint32_t ko = ks * 32;
-            umma_f16_2cta(d, umma_desc_sw128(xlo + ko), umma_desc_sw128(whi + ko), IDESC, (kc == 0 && ks == 0) ? 0u : 1u);
-            umma_f16_2cta(d, umma_desc_sw128(xhi + ko), umma_desc_sw128(wlo + ko), IDESC, 1u);
-            umma_f16_2cta(d, umma_desc_sw128(xhi + ko), umma_desc_sw128(whi + ko), IDESC, 1u);
-          }
-          umma_commit_2cta(&ctl->empty[s]);
-        }
-        umma_commit_2cta(&ctl->acc_full[j & 1]);
-      }
-    } else if (lane == 0) {
-      const uint32_t total = (uint32_t)n_my * C2;        // peer: forward "my stage has landed" to the leader
-      for (uint32_t gw = 0; gw < total; ++gw) {
-        const uint32_t s = gw % PG_STAGES;
-        mbar_wait(&ctl->full[s], (gw / PG_STAGES) & 1);
-        mbar_arrive_cluster(l_peer + 8u * s);
-      }
-    }
-    __syncwarp();
-  } else {
-    if (lane == 0) {
-      uint32_t gw = 0;
-      for (int j = 0; j < n_my; ++j) {
-        int mp, nt;
-        item(pair + j * npairs, mp, nt);
-        const char* a = g.himg + (size_t)(2 * mp + rank) * (size_t)(C2 * SLOT_BYTES);
-        const float* hi = g.Whi + (size_t)nt * C2 * G::B_CHUNK_FLOATS + (size_t)rank * (HB / 4);
-        const float* lo = g.Wlo + (size_t)nt * C2 * G::B_CHUNK_FLOATS + (size_t)rank * (HB / 4);
-        for (int kc = 0; kc < C2; ++kc, ++gw) {
-          const int s = gw % PG_STAGES;
-          mbar_wait(&ctl->empty[s], ((gw / PG_STAGES) & 1) ^ 1);
-          char* dst = ring + (size_t)s * STAGE;
-          mbar_arrive_expect_tx(&ctl->full[s], STAGE);
-          bulk_g2s(dst, a + (size_t)kc * SLOT_BYTES, SLOT_BYTES, &ctl->full[s]);
-          bulk_g2s(dst + SLOT_BYTES, hi + (size_t)kc * G::B_CHUNK_FLOATS, HB, &ctl->full[s]);
-          bulk_g2s(dst + SLOT_BYTES + HB, lo + (size_t)kc * G::B_CHUNK_FLOATS, HB, &ctl->full[s]);
-        }
-      }
-    }
-    __syncwarp();
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == PG_MMA) tmem_dealloc2(ctl->tmem_base, 512);
-}
-
-// =====================================================================================================
 // edge kernels
 // =====================================================================================================
-// unroll factors of the epilogue loops (overridable for tuning builds: -DDSB_E1_UNROLL=... etc.)
-#ifndef DSB_E1_UNROLL
-#define DSB_E1_UNROLL 2
-#endif
-#ifndef DSB_E2_UNROLL
-#define DSB_E2_UNROLL 2
-#endif
-constexpr int kE1Unroll = DSB_E1_UNROLL, kE2Unroll = DSB_E2_UNROLL;
-#ifndef DSB_EARLY_UNIT
-#define DSB_EARLY_UNIT 0        // edge producers: 1 = next unit's first gathers issued during the last half of the current unit
-                                // (measured: GCL 133.2 vs 132.6 us, coord 63.8 vs 61.7 us per launch with 0 -> off)
-#endif
-#ifndef DSB_RED_PAIR
-#define DSB_RED_PAIR 1          // GCL pass 2: one RED per chunk PAIR of the same receiver
-#endif
+constexpr int kE1Unroll = 2, kE2Unroll = 2;   // unroll factors of the epilogue's pass-1 and pass-2 loops
 constexpr int EPI_T_STRIDE = 36;          // 16-byte aligned rows: conflict-free row-wise STS.128 and column-wise LDS.32
 constexpr int NSCAL = 3;                   // scalar buffer sets (the j-th tile of a CTA uses set j % NSCAL)
 constexpr int SCAL_WARPS = 2;              // warps 14, 15 of the edge kernels: per-edge scalars one tile ahead of the producers
@@ -1464,7 +1197,7 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
             a01 = add2(pk2(v[4 * q], v[4 * q + 1]), pk2(bb.x, bb.y));
             a23 = add2(pk2(v[4 * q + 2], v[4 * q + 3]), pk2(bb.z, bb.w));
           }
-          silu_pair<(DSB_SILU_PAIR & 2) != 0, (DSB_SILU_QUAD & 2) != 0>(a01, a23);
+          silu4q(a01, a23);
           upk2(a01, v[4 * q], v[4 * q + 1]); upk2(a23, v[4 * q + 2], v[4 * q + 3]);
           s01 = fma2(a01, pk2(ww.x, ww.y), s01); s23 = fma2(a23, pk2(ww.z, ww.w), s23);
         }
@@ -1487,7 +1220,6 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
         float* G4 = ex->gate4[warp];
         G4[lane] = gate;
         __syncwarp();
-#if DSB_RED_PAIR
         // lane (rg = lane / 8, cg = lane % 8) owns the chunk PAIR of rows 8 rg .. 8 rg + 7 x columns 4 cg .. 4 cg + 3 of the block:
         // 8 LDS.128 (one row each; the quarter-warp reads 128 contiguous bytes of a row), the two gate-weighted chunk sums,
         // and ONE 16-byte RED when both chunks belong to the same receiver (3 of 4 pairs at ~24 edges per receiver; a chunk of
@@ -1529,39 +1261,6 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
           }
           __syncwarp();
         }
-#else
-        const int ck = lane >> 2, cg = lane & 3;
-        const float4 gq = *reinterpret_cast<const float4*>(G4 + 4 * ck);         // gates of the chunk's four rows
-        const f32x2 g0 = pk2(gq.x, gq.x), g1 = pk2(gq.y, gq.y), g2 = pk2(gq.z, gq.z), g3 = pk2(gq.w, gq.w);
-        const int crow = max(ex->row[par][warp * 32 + 4 * ck], 0);
-        float* const dst0 = a.agg + (size_t)crow * H + 4 * cg;
-        const float* const tp = T + (4 * ck) * EPI_T_STRIDE + 4 * cg;
-#pragma unroll kE2Unroll
-        for (int cb = 0; cb < ((edbg & 16) ? 0 : TN / 32); ++cb) {
-          float v[32];
-          tmem_ld32(taddr + cb * 32, v);
-#pragma unroll
-          for (int q = 0; q < 8; ++q)
-            *reinterpret_cast<float4*>(T + lane * EPI_T_STRIDE + 4 * q) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-          __syncwarp();
-          if (!(edbg & 1024)) {
-#pragma unroll
-            for (int hp = 0; hp < 2; ++hp) {
-              const float4 x0 = *reinterpret_cast<const float4*>(tp + 16 * hp);
-              const float4 x1 = *reinterpret_cast<const float4*>(tp + 16 * hp + EPI_T_STRIDE);
-              const float4 x2 = *reinterpret_cast<const float4*>(tp + 16 * hp + 2 * EPI_T_STRIDE);
-              const float4 x3 = *reinterpret_cast<const float4*>(tp + 16 * hp + 3 * EPI_T_STRIDE);
-              // ((g0 x0 + g1 x1) + (g2 x2 + g3 x3)): two independent chains per pair
-              const f32x2 s01 = add2(fma2(g1, pk2(x1.x, x1.y), mul2(g0, pk2(x0.x, x0.y))), fma2(g3, pk2(x3.x, x3.y), mul2(g2, pk2(x2.x, x2.y))));
-              const f32x2 s23 = add2(fma2(g1, pk2(x1.z, x1.w), mul2(g0, pk2(x0.z, x0.w))), fma2(g3, pk2(x3.z, x3.w), mul2(g2, pk2(x2.z, x2.w))));
-              float o0, o1, o2, o3;
-              upk2(s01, o0, o1); upk2(s23, o2, o3);
-              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst0 + cb * 32 + 16 * hp), "f"(o0), "f"(o1), "f"(o2), "f"(o3) : "memory");
-            }
-          }
-          __syncwarp();
-        }
-#endif
       } else {
         // coord: s = phi_m for this edge row; this unit's term of trans (egnn_new.py:100-109)
         const int r = warp * 32 + lane;
@@ -1659,12 +1358,6 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
         if (TB) pty[i] = ex->type[par][r0 + i] * H;
       }
     };
-    // (iii) early (DSB_EARLY_UNIT, off): with an even number of chunks the register set the next unit's chunk 0 reads (set 0) is
-    // idle during the last chunk (set 1), and the row pointers are dead after the last half's loads, so the next unit's first
-    // gathers could go out a whole half before the unit boundary instead of right in front of their first use (6 % of the
-    // producers' samples are that stall) - but the producers have slack (they wait 17 % of their time for the ring) and the
-    // longer live ranges cost more than the stall: slower when measured.
-    constexpr bool kEarlyUnit = DSB_EARLY_UNIT && (chunks % 2 == 0);
     const bool no_gather = (dbg & 64) != 0;        // instrumented builds only: operands from registers instead of L2
     auto ld4 = [&](const float* p) { return no_gather ? make_float4(0.1f, -0.2f, 0.3f, 0.05f) : *reinterpret_cast<const float4*>(p); };
     auto issue = [&](int hf, float4& xa, float4 (&xb)[4]) {
@@ -1674,7 +1367,7 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
     };
     long long t0 = 0, t1 = 0, t2 = 0, acc_wait = 0, acc_comp = 0, acc_fence = 0;
     const long long pp0 = pprof ? tc_clock() : 0;
-    int m = setup_ptrs(0), m_next = 0;
+    int m = setup_ptrs(0);
     setup_scal(0);
     issue(0, GA[0], GB[0]);
     for (int j = 0; j < n_my; ++j) {
@@ -1694,10 +1387,6 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
           const int hf = kc * HPC + h;
           const bool last_half = (h == HPC - 1);
           if (last_half && kc + 1 < chunks && !(dbg & 2)) issue(hf + 1, GA[(kc & 1) ^ 1], GB[(kc & 1) ^ 1]);          // (ii)
-          if (kEarlyUnit && last_half && kc + 1 == chunks && j + 1 < n_my) {                                         // (iii) early
-            m_next = setup_ptrs(j + 1);
-            if (!(dbg & 2)) issue(0, GA[0], GB[0]);
-          }
           if (!(dbg & 2)) {
             const float4 r4 = *reinterpret_cast<const float4*>(wr + hf * TKC);
             const float4 r04 = *reinterpret_cast<const float4*>(wr0 + hf * TKC);
@@ -1713,7 +1402,7 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
                 const float4 t4 = *reinterpret_cast<const float4*>(tbm + pty[i] + hf * TKC);
                 u01 = add2(u01, pk2(t4.x, t4.y)); u23 = add2(u23, pk2(t4.z, t4.w));
               }
-              if (!(dbg & 128)) silu_pair<(DSB_SILU_PAIR & 1) != 0, (DSB_SILU_QUAD & 1) != 0>(u01, u23);      // 128: instrumented builds only
+              if (!(dbg & 128)) silu4q(u01, u23);      // 128: instrumented builds only
               store_pair<F16>(st + (F16 && (hf & 1) ? (so[i] ^ 64u) : so[i]), u01, u23);
             }
           }
@@ -1726,11 +1415,8 @@ __global__ void __launch_bounds__(EDGE_THREADS, 1) tc_edge_kernel(TcEdgeArgs a) 
         if (pprof) acc_fence += tc_clock() - t2;
       }
       if (j + 1 < n_my) {                                                                      // (iii)
-        if (kEarlyUnit) m = m_next;
-        else {
-          m = setup_ptrs(j + 1);
-          if (!(dbg & 2)) issue(0, GA[0], GB[0]);
-        }
+        m = setup_ptrs(j + 1);
+        if (!(dbg & 2)) issue(0, GA[0], GB[0]);
         setup_scal(j + 1);
       }
       if (pprof) {
@@ -1826,13 +1512,11 @@ template <int H, bool PAIR> static size_t edge_smem_bytes() {
   return edge_smem_base<H, PAIR>() + sizeof(EdgeExtra<H>);
 }
 // Kernel-form selection (dsb_set_kernel_variants): bit 0 = CTA-pair weight-stationary edge kernels, bit 1 = fused node block
-// kernel, bit 2 = its phase 3 as a separate CTA-pair GEMM (off by default: measured equal, one launch more).  3xTF32 always
-// uses the single-CTA kernels.
+// kernel.  3xTF32 always uses the single-CTA kernels.
 int g_kernel_variants = [] {
   int v = 3;
   const char* e = getenv("DSB_EDGE_PAIR"); if (e && e[0] == '0') v &= ~1;
   e = getenv("DSB_NODE_BLOCK"); if (e && e[0] == '0') v &= ~2;
-  e = getenv("DSB_NODE_SPLIT"); if (e && e[0] == '1') v |= 4;
   return v;
 }();
 static bool edge_pair_enabled() { return (g_kernel_variants & 1) != 0; }
@@ -1859,8 +1543,6 @@ int configure_tc_kernels(int H) {
     DSB_CUDA_OK(cudaFuncSetAttribute(tc_node_gemm_kernel<true, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, gs));
     static_assert(block_smem_bytes<W>() <= 232448, "node block kernel exceeds shared memory");
     DSB_CUDA_OK(cudaFuncSetAttribute(tc_node_block_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)block_smem_bytes<W>()));
-    static_assert(pair_gemm_smem_bytes<W>() <= 232448, "pair GEMM exceeds shared memory");
-    DSB_CUDA_OK(cudaFuncSetAttribute(tc_pair_gemm_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair_gemm_smem_bytes<W>()));
     DSB_CUDA_OK(cudaFuncSetAttribute(tc_edge_kernel<false, false, W, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, es));
     DSB_CUDA_OK(cudaFuncSetAttribute(tc_edge_kernel<false, false, W, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, es));
     DSB_CUDA_OK(cudaFuncSetAttribute(tc_edge_kernel<false, true, W, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, es));
@@ -1877,21 +1559,22 @@ int configure_tc_kernels(int H) {
   });
 }
 
-int launch_tc_node_gemm(const dsb_dynamics* d, const GemmArgs& g, const TcImage& w, int n_tile_off, bool f16, int32_t* status,
-                        cudaStream_t s) {
+int launch_tc_node_gemm(const dsb_dynamics* d, const GemmArgs& g, const TcImage& w, bool f16, int32_t* status, cudaStream_t s) {
   if (g.M == 0) return 0;
-  const int K = g.K1 + g.K2, TN = d->cfg.hidden_nf;
-  if ((g.Nn % TN) || (K % TKC16) || (g.K1 % TKC16) || (g.lda1 % 4) || (g.ldc % 4)) {
-    set_error("tc_node_gemm: unsupported shape K1=%d K2=%d Nn=%d", g.K1, g.K2, g.Nn);
+  const int TN = d->cfg.hidden_nf;
+  if (g.A2 || g.K2 || !g.bias || g.R || g.act || g.Z) {
+    set_error("tc_node_gemm computes C = A W + bias only (no second operand, activation, residual or zeroing)");
+    return DSB_ERR_INVALID_ARGUMENT;
+  }
+  if ((g.Nn % TN) || (g.K1 % TKC16) || (g.lda1 % 4) || (g.ldc % 4)) {
+    set_error("tc_node_gemm: unsupported shape K=%d Nn=%d", g.K1, g.Nn);
     return DSB_ERR_INVALID_ARGUMENT;
   }
   TcGemmArgs a;
-  a.A1 = g.A1; a.lda1 = g.lda1; a.K1 = g.K1; a.A2 = g.A2; a.lda2 = g.lda2; a.K2 = g.K2; a.div2 = g.div2; a.deg2 = g.deg2;
-  const size_t img_off = (size_t)n_tile_off * (K / (f16 ? TKC16 : TKC)) * (size_t)(TN * TKC);     // skip the first n-tiles of the image
-  a.Bhi = (f16 ? w.h_hi : w.t_hi) + img_off; a.Blo = (f16 ? w.h_lo : w.t_lo) + img_off;
-  a.Z = g.Z; a.ldz = g.ldz;
+  a.A = g.A1; a.lda = g.lda1; a.K = g.K1;
+  a.Bhi = f16 ? w.h_hi : w.t_hi; a.Blo = f16 ? w.h_lo : w.t_lo;
   a.dead_nt = g.dead_cols / TN; a.dead_mt = a.dead_nt > 0 ? (g.dead_rows_from + TM - 1) / TM : 0;
-  a.bias = g.bias; a.R = g.R; a.ldr = g.ldr; a.C = g.C; a.ldc = g.ldc; a.M = g.M; a.Nn = g.Nn; a.act = g.act;
+  a.bias = g.bias; a.C = g.C; a.ldc = g.ldc; a.M = g.M; a.Nn = g.Nn;
   a.inv_scale = f16 ? w.h_inv : 1.0f; a.status = status;
   const int ntn_ = g.Nn / TN, ntm_ = (g.M + TM - 1) / TM;
   const int dmt_ = a.dead_nt > 0 ? (a.dead_mt < ntm_ ? a.dead_mt : ntm_) : ntm_;
@@ -1942,16 +1625,8 @@ int launch_tc_node_block(const dsb_dynamics* d, const Dims& dm, const Workspace&
   if (a.Nn % H) { set_error("tc_node_block: %d output columns are not a multiple of hidden_nf", a.Nn); return DSB_ERR_INVALID_ARGUMENT; }
   const int ntm = (dm.N + TM - 1) / TM, nmp = (ntm + 1) / 2, hw = d->num_sms / 2;
   const int grid = 2 * (nmp < hw ? nmp : hw);
-  const bool split = (g_kernel_variants & 4) != 0;      // phase 3 as a separate, evenly loaded CTA-pair GEMM from the operand image of h
-  a.himg = split ? reinterpret_cast<char*>(ws.hT) : nullptr;
   return dispatch_width(H, [&]<int W>() -> int {
     DSB_CUDA_OK(launch_k_pair(tc_node_block_kernel<W>, grid, TC_THREADS, block_smem_bytes<W>(), s, a));
-    if (split) {
-      TcPairGemmArgs b = {};
-      b.himg = a.himg; b.Whi = a.Wqhi; b.Wlo = a.Wqlo; b.bias = a.bq; b.inv = a.invq;
-      b.C = P; b.ldc = ldp; b.M = dm.N; b.Nn = a.Nn; b.dead_mt = a.dead_mt; b.dead_nt = a.dead_nt;
-      DSB_CUDA_OK(launch_k_pair(tc_pair_gemm_kernel<W>, 2 * hw, PG_THREADS, pair_gemm_smem_bytes<W>(), s, b));
-    }
     return 0;
   });
 }

@@ -318,32 +318,15 @@ __device__ __forceinline__ void store_piece(char* st, int row, int half, int p, 
 }
 
 // Same split as store_piece, for a row piece already held as two packed pairs and a precomputed destination address
-// (stage base + swizzled offset of the row piece): the residual is one packed subtraction.
-__device__ __forceinline__ f32x2 sub2_(f32x2 a, f32x2 b) { f32x2 r; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b)); return r; }
-#ifndef DSB_SPLIT_TRUNC
-#define DSB_SPLIT_TRUNC 0
-#endif
+// (stage base + swizzled offset of the row piece).
 template <bool F16>
 __device__ __forceinline__ void store_pair(char* dst, f32x2 u01, f32x2 u23) {
   float x0, x1, x2, x3;
   upk2(u01, x0, x1); upk2(u23, x2, x3);
   if constexpr (F16) {
-#if DSB_SPLIT_TRUNC
-    // hi = x with the 13 low mantissa bits cleared (exactly representable in fp16 when normal there): four LOP3 on the ALU pipe
-    // instead of four half->float conversions on the FMA pipe; the residual is < 2^-10 |x| (rounding: 2^-11), kept to 11 bits
-    const float t0 = __uint_as_float(__float_as_uint(x0) & 0xffffe000u), t1 = __uint_as_float(__float_as_uint(x1) & 0xffffe000u);
-    const float t2 = __uint_as_float(__float_as_uint(x2) & 0xffffe000u), t3 = __uint_as_float(__float_as_uint(x3) & 0xffffe000u);
-    const __half2 h0 = __floats2half2_rn(t0, t1), h1 = __floats2half2_rn(t2, t3);
-    const float2 f0 = make_float2(t0, t1), f1 = make_float2(t2, t3);
-#else
     const __half2 h0 = __floats2half2_rn(x0, x1), h1 = __floats2half2_rn(x2, x3);
-#endif
     float l0, l1, l2, l3;
-#if DSB_SPLIT_TRUNC
-    upk2(sub2_(u01, pk2(f0.x, f0.y)), l0, l1); upk2(sub2_(u23, pk2(f1.x, f1.y)), l2, l3);
-#else
     residual_f16(h2_bits(h0), x0, x1, l0, l1); residual_f16(h2_bits(h1), x2, x3, l2, l3);
-#endif
     const __half2 q0 = __floats2half2_rn(l0, l1), q1 = __floats2half2_rn(l2, l3);
     uint2 hv, lv;
     hv.x = *reinterpret_cast<const uint32_t*>(&h0); hv.y = *reinterpret_cast<const uint32_t*>(&h1);

@@ -134,10 +134,8 @@ int dsb_set_programmatic_launch(int enable);
 /* Process-wide selection among equivalent kernel forms of the 3xFP16 path (same results within the parity tolerance).
  * Bit 0: the edge kernels run as CTA pairs (tcgen05 cta_group::2) with the second-layer weights resident in shared memory
  * instead of single CTAs that stream them; bit 1: node_model and the merged first-layer GEMM of a block run as one fused
- * CTA-pair kernel instead of two launches; bit 2: that kernel stops after the node update and the merged GEMM runs as a
- * separate, evenly loaded CTA-pair GEMM fed by bulk copies of an operand image of h.  variants < 0 = query only.  Returns
- * the previous setting.  Initial value: 3 (bit 2 measured equal to the fused form, one launch more), minus bit 0 / 1 if the
- * environment has DSB_EDGE_PAIR=0 / DSB_NODE_BLOCK=0, plus bit 2 if DSB_NODE_SPLIT=1. */
+ * CTA-pair kernel instead of two launches.  Higher bits are ignored.  variants < 0 = query only.  Returns the previous
+ * setting.  Initial value: 3, minus bit 0 / 1 if the environment has DSB_EDGE_PAIR=0 / DSB_NODE_BLOCK=0. */
 int dsb_set_kernel_variants(int variants);
 
 /* ---- arithmetic path.  mode is a bitmask: 1 = node GEMMs, 2 = edge (GCL) kernel, 4 = coordinate edge kernel run on

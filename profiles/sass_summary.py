@@ -14,7 +14,7 @@ from diffsbdd_b200 import _build  # noqa: E402
 KEYS = ['UTCHMMA.2CTA', 'UTCHMMA', 'UTCBAR.2CTA.MULTICAST', 'UTCBAR', 'LDTM', 'STTM', 'UBLKCP', 'UTMALDG', 'UCGABAR_ARV', 'SYNCS', 'FENCE.VIEW.ASYNC',
         'USETMAXREG', 'FHFMA', 'HADD2.F32', 'MUFU.EX2', 'MUFU.RCP', 'FFMA2', 'FADD2', 'FMUL2', 'F2FP', 'REDG.E.ADD.F32x4', 'REDG', 'LDG.E.128', 'STS.64', 'STS.128', 'LDS.128']
 WANT = ['tc_edge_kernelILb0ELb1ELi256ELb0ELb1', 'tc_edge_kernelILb1ELb1ELi256ELb0ELb1', 'tc_edge_kernelILb0ELb1ELi256ELb0ELb0',
-        'tc_node_block_kernelILi256', 'tc_pair_gemm_kernelILi256', 'tc_node_gemm_kernelILb1ELi256', 'tc_node_mlp_kernelILb1ELi256']
+        'tc_node_block_kernelILi256', 'tc_node_gemm_kernelILb1ELi256', 'tc_node_mlp_kernelILb1ELi256']
 out = subprocess.run(['cuobjdump', '-sass', _build.LIB_PATH], capture_output=True, text=True).stdout
 cur, counts = None, collections.OrderedDict()
 for line in out.splitlines():

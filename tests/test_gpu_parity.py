@@ -309,7 +309,7 @@ def test_single_cta_kernel_forms_still_match():
         a = run(net, inp)
         assert_close(a[0], want[0], 'single-CTA forms, ligand out')
         assert_close(a[1], want[1], 'single-CTA forms, pocket out')
-        for v in (1, 2, 6, 7):
+        for v in (1, 2):
             lib.dsb_set_kernel_variants(v)
             b = run(net, inp)
             assert_close(b[0], want[0], f'kernel variants {v}, ligand out')
